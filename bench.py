@@ -25,6 +25,9 @@ rank keeps 64 images).  Prints ONE JSON line on rank 0.
              the N-rank sums equal the sums of a single rank that ran every image (bit for bit, fp64)
   --impl reference : times ONLY that CPU implementation (the reference is pure Python on PyTorch;
              /root/reference does not exist on the GPU box, so the oracle port stands in).
+  --dump-outputs DIR : after the timed steps, writes the depth maps the timed path returned in its last step (rank 0) as
+             DIR/depth.npy (float32).  Inputs and weights are seeded, so two builds run with the same arguments can be
+             compared output for output.
 """
 import argparse
 import json
@@ -64,6 +67,7 @@ def parse():
     ap.add_argument('--e2e-steps', type=int, default=200)
     ap.add_argument('--lanes', type=int, default=3, help='batches in flight: independent plan copies on their own streams '
                                                          '(fastdepth_b200.engine.ForwardLanes); 1 = strict single stream')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the last timed step\'s depth maps to DIR/depth.npy')
     return ap.parse_args()
 
 
@@ -78,6 +82,19 @@ def peaks():
 
 
 NOMINAL_HBM_GBS = 8000.0        # the figure north_star quotes
+DUMP_MAX_ELEMS = 12 << 20       # 48 MiB of float32: keeps a dump well under 64 MB
+
+
+def dump_outputs(out_dir, y):
+    """Write ``y`` as out_dir/depth.npy in float32.  An output of more than DUMP_MAX_ELEMS elements is replaced by a fixed sample:
+    the flattened elements at DUMP_MAX_ELEMS positions drawn with a fixed seed (the same positions for the same shape)."""
+    import numpy as np
+    a = y.detach().float().cpu().numpy()
+    if a.size > DUMP_MAX_ELEMS:
+        pos = np.sort(np.random.Generator(np.random.PCG64(0)).choice(a.size, size=DUMP_MAX_ELEMS, replace=False))
+        a = a.reshape(-1)[pos]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'depth.npy'), a)
 
 
 def eager_reference_forward(model, x):
@@ -227,7 +244,7 @@ def pick_cpu_threads(sd, h, w):
 
 
 def cpu_forward_rate(sd, h, w, budget_s, min_steps, warmup, batch=None):
-    """Time the oracle port of the reference forward on the host cores; returns (img/s, batch, steps, s/step)."""
+    """Time the oracle port of the reference forward on the host cores; returns (img/s, batch, steps, s/step, last output)."""
     from fastdepth_b200 import synthetic
     from oracle import fastdepth_oracle as orc          # the CPU baseline leg may execute the oracle
     torch.set_grad_enabled(False)
@@ -243,12 +260,12 @@ def cpu_forward_rate(sd, h, w, budget_s, min_steps, warmup, batch=None):
     t_start = time.perf_counter()
     while len(times) < min_steps or (budget_s and time.perf_counter() - t_start < budget_s and len(times) < 10 * min_steps):
         t0 = time.perf_counter()
-        orc.skipadd_forward(sd, x)
+        y = orc.skipadd_forward(sd, x)
         times.append(time.perf_counter() - t0)
         if budget_s and time.perf_counter() - t_start > budget_s and len(times) >= min_steps:
             break
     per = sum(times) / len(times)
-    return batch / per, batch, len(times), per
+    return batch / per, batch, len(times), per, y
 
 
 def run_eval(rank, world, dev, widths, sd, h, w, n, lanes=1):
@@ -328,7 +345,9 @@ def run_reference(args, rank):
     cores, thread_note = pick_cpu_threads(sd, h, w)
     # batch <= 8 per step on purpose: that is where the CPU forward is fastest per image (batch 64 measured 31 img/s against 77-240
     # at batch 8 on the same cores: the activations fall out of the caches), and the reference arm should be the reference at its best
-    rate, batch, steps, per = cpu_forward_rate(sd, h, w, budget_s=0, min_steps=max(1, args.steps), warmup=max(1, args.warmup))
+    rate, batch, steps, per, y = cpu_forward_rate(sd, h, w, budget_s=0, min_steps=max(1, args.steps), warmup=max(1, args.warmup))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y)
     line = {
         'impl': 'reference', 'metric': METRIC, 'value': rate, 'unit': UNIT, 'n_gpus': args.gpus, 'steps': steps,
         'warmup': max(1, args.warmup), 'ms_per_step': per * 1e3, 'higher_is_better': True, 'scaling': 'weak',
@@ -429,6 +448,8 @@ def main():
                          args.steps, max(3, args.warmup) * R, fan=lane_streams)
     else:
         ms_total = ms_single
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, lane_y[(args.steps - 1) % R] if R > 1 else y)
     # ---- e2e: pinned host buffers through the C-ABI pipeline (fd_pipeline_submit / fd_pipeline_wait): every step
     # uploads its batch from pinned host memory and downloads its depth maps; up to 3 batches are in flight so
     # the PCIe copies overlap the forward of the neighbouring steps.  Timed on the host clock between device-wide
@@ -529,7 +550,7 @@ def main():
     cpu = None
     if not args.no_cpu_baseline and world == 1:
         ccores, thread_note = pick_cpu_threads(sd, h, w)
-        rate, cb, csteps, per = cpu_forward_rate(sd, h, w, budget_s=15.0, min_steps=3, warmup=1)
+        rate, cb, csteps, per, _ = cpu_forward_rate(sd, h, w, budget_s=15.0, min_steps=3, warmup=1)
         cpu = {'value': rate, 'unit': UNIT, 'cores': ccores, 'kind': 'port',
                'sample': '%d forwards of batch %d at %dx%d, fp32 torch CPU (oracle port of reference models.py:706-732), '
                          '%.2f s each; %s' % (csteps, cb, h, w, per, thread_note)}
